@@ -494,9 +494,47 @@ class _Raw:
         self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 3}
 
 
-def gpu_workload(name, args, env, units, steps, warmup, with_e2e=False):
+DUMP_SAMPLE_UNITS = 1 << 18       # per-read records of this many units (seeded sample, sorted indices) go into the dump
+
+
+def dump_outputs(path, torch, capi, n, cnt, out1, out2, ov, patches, npatch):
+    """Write what the last timed pass handed back to its caller as DIR/<name>.npy (float32, float64 where an integer can pass
+    2**24): the whole counter block, every field of the per-read and overlap records of a fixed sample of units, and the
+    correction patches of those units sorted by (unit, read, position).  Two builds run with the same arguments see the same
+    inputs, so their dumps compare array for array."""
+    os.makedirs(path, exist_ok=True)
+    m = min(n, DUMP_SAMPLE_UNITS)
+    idx = np.sort(np.random.default_rng(SEED).choice(n, size=m, replace=False))
+    it = torch.from_numpy(idx).to(out1.device)
+    arrays = {"sample_index": idx.astype(np.float64), "counters": cnt.astype(np.float64)}
+    for tag, buf, dt in (("out1", out1, capi.READ_RESULT_DTYPE), ("out2", out2, capi.READ_RESULT_DTYPE), ("ov", ov, capi.OV_RESULT_DTYPE)):
+        if buf is None:
+            continue
+        rec = buf.view(n, dt.itemsize)[it].cpu().numpy().view(dt).reshape(m)
+        for f in dt.names:
+            if f != "reserved":
+                arrays[f"{tag}_{f}"] = rec[f].astype(np.float32)
+    if patches is not None:
+        k = int(npatch.item())
+        rows = patches[: min(k, patches.numel() // 12) * 12].view(-1, 12)
+        keep = torch.zeros(n, dtype=torch.bool, device=out1.device)
+        keep[it] = True
+        rows = rows[keep[rows[:, :4].contiguous().view(torch.int32).view(-1).long()]]
+        pt = np.sort(rows.cpu().numpy().view(capi.PATCH_DTYPE).reshape(-1), order=["pair", "which", "pos"])
+        arrays["patch_count"] = np.array([k], np.float64)
+        arrays["patch_unit"] = pt["pair"].astype(np.float64)
+        for f in ("pos", "which", "base", "qual", "old_base", "old_qual"):
+            arrays[f"patch_{f}"] = pt[f].astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"dump of {total} bytes"
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def gpu_workload(name, args, env, units, steps, warmup, with_e2e=False, dump_dir=None):
     """W warm-up + K timed passes of one BASELINE config over a batch resident in HBM; returns the result dict
-    (value, roofline, checks, ...).  env: torch, dist, capi, lib, world, rank, local_rank, dev, comm."""
+    (value, roofline, checks, ...).  env: torch, dist, capi, lib, world, rank, local_rank, dev, comm.
+    dump_dir: write the outputs of the last timed pass there (dump_outputs)."""
     torch, dist, capi, lib = env["torch"], env["dist"], env["capi"], env["lib"]
     world, rank, local_rank, dev = env["world"], env["rank"], env["local_rank"], env["dev"]
     W = WORKLOADS[name]
@@ -508,6 +546,9 @@ def gpu_workload(name, args, env, units, steps, warmup, with_e2e=False):
     free_b, _ = torch.cuda.mem_get_info()
     per_unit = sides * (2 * S + 2 + 16) + (8 + 15 if paired else 0)
     n = int(min(units, 0.85 * free_b / per_unit))
+    if dump_dir is not None and n < units:
+        raise SystemExit(f"bench.py --dump-outputs: {units} units do not fit in free device memory ({free_b / 1e9:.1f} GB); "
+                         "a smaller batch would change the inputs")
     first = rank * n                                   # rank r owns global indices [r*n, (r+1)*n)
 
     def alloc(nbytes):
@@ -621,6 +662,8 @@ def gpu_workload(name, args, env, units, steps, warmup, with_e2e=False):
     cnt = np.zeros(Lc.total, np.int64)
     capi.check(lib.fp_counters_fetch(h, cnt.ctypes.data), lib)
     cv = capi.CounterView(Lc, cnt)
+    if dump_dir is not None and rank == 0:     # before the parity pass below overwrites the records and the counter block
+        dump_outputs(dump_dir, torch, capi, n, cnt, out1, out2, ov, patches, npatch)
     total_units = n * world
     checks = {
         "pre_reads_eq_units": bool(cv.stats(capi.STATS_PRE1)["reads"] == total_units),
@@ -897,6 +940,8 @@ def main():
     ap.add_argument("--no-workloads", action="store_true", help="skip the other BASELINE configs (the `workloads` object)")
     ap.add_argument("--fastq-units", type=int, default=1_000_000,
                     help="units of the text-in/text-out measurement (device FASTQ decode + chain + encode); 0 = skip")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of --workload as DIR/<name>.npy (counter block, records of a seeded sample of units)")
     args = ap.parse_args()
 
     if args.impl == "reference":
@@ -968,7 +1013,8 @@ def main():
         units = (args.units or WORKLOADS[nm]["units"]) if main_wl else min(args.units or WORKLOADS[nm]["units"], WORKLOADS[nm]["units"])
         try:
             res, parity, _ = gpu_workload(nm, args, env, units, args.steps if main_wl else max(2, min(args.steps, 3)),
-                                          args.warmup if main_wl else 3, with_e2e=main_wl and not args.no_e2e)
+                                          args.warmup if main_wl else 3, with_e2e=main_wl and not args.no_e2e,
+                                          dump_dir=args.dump_outputs if main_wl else None)
         except Exception as e:
             if main_wl:
                 raise

@@ -11,4 +11,4 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs oracle/_ref (built from /root/reference)")
+    config.addinivalue_line("markers", "reference: compares with the reference's answers (oracle/_ref where built, else tests/golden/reference_digests.json)")

@@ -1,6 +1,8 @@
 """Test infrastructure: loaders for the CPU checkers under oracle/ and comparison helpers.
 Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs may use oracle/."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -76,6 +78,108 @@ def ref():
         lib.fp_ref_process_mt.argtypes = _PROC_ARGS + [C.c_int]
         _ref = lib
     return _ref
+
+
+# ---------------- the reference's answers, stored as digests ----------------
+# oracle/_ref is built only where the reference sources are.  Every comparison with it is therefore pinned by the digests of the
+# reference's answers in REF_DIGESTS: without the build the tested value must hash to them; with it the reference runs as well,
+# its answer must still hash to them (FP_UPDATE_GOLDEN=1 rewrites them instead) and the tested value must equal it.
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "reference_digests.json")
+_digests = None
+
+
+def _feed(h, o):
+    if isinstance(o, np.ndarray):
+        h.update(repr((o.dtype.str, o.shape)).encode())
+        h.update(np.ascontiguousarray(o).tobytes())
+    elif isinstance(o, dict):
+        h.update(b"{%d" % len(o))
+        for k in sorted(o):
+            _feed(h, k); _feed(h, o[k])
+    elif isinstance(o, (list, tuple)):
+        h.update(b"[%d" % len(o))
+        for x in o:
+            _feed(h, x)
+    elif isinstance(o, bytes):
+        h.update(b"b%d:" % len(o)); h.update(o)
+    else:
+        h.update(repr(o.item() if isinstance(o, np.generic) else o).encode())
+
+
+def digest(obj):
+    h = hashlib.sha256()
+    _feed(h, obj)
+    return h.hexdigest()[:12]
+
+
+def _digest_of(obj):
+    return {k: digest(v) for k, v in obj.items()} if isinstance(obj, dict) else digest(obj)
+
+
+def _assert_same(got, want, what):
+    if isinstance(want, dict):
+        assert sorted(got) == sorted(want), f"{what}: keys {sorted(got)} vs {sorted(want)}"
+        for k in want:
+            _assert_same(got[k], want[k], f"{what}.{k}")
+    elif isinstance(want, np.ndarray):
+        assert got.shape == want.shape, f"{what}: shape {got.shape} vs {want.shape}"
+        i = np.argwhere(got != want)
+        assert i.size == 0, f"{what} differs at {tuple(i[0])}: {got[tuple(i[0])]} vs {want[tuple(i[0])]}"
+    else:
+        assert got == want, f"{what}: {got!r} vs {want!r}"
+
+
+def check_reference(key, got, reference):
+    """Assert that `got` equals the reference's answer for case `key`; reference() computes that answer with oracle/_ref.
+    A dict is pinned key by key, so a failure names the field."""
+    global _digests
+    if _digests is None:
+        _digests = json.load(open(REF_DIGESTS)) if os.path.exists(REF_DIGESTS) else {}
+    if have_ref():
+        want = reference()
+        if os.environ.get("FP_UPDATE_GOLDEN") == "1":
+            _digests[key] = _digest_of(want)
+            with open(REF_DIGESTS, "w") as f:
+                json.dump(_digests, f, indent=0, sort_keys=True)
+                f.write("\n")
+        else:
+            assert _digest_of(want) == _digests.get(key), f"{key}: the reference's answer no longer matches {REF_DIGESTS} (FP_UPDATE_GOLDEN=1 rewrites it)"
+        _assert_same(got, want, key)
+        return
+    assert key in _digests, f"{key}: no stored reference answer in {REF_DIGESTS}"
+    stored, mine = _digests[key], _digest_of(got)
+    if isinstance(stored, dict):
+        assert sorted(mine) == sorted(stored), f"{key}: fields {sorted(mine)} vs {sorted(stored)}"
+        bad = [k for k in stored if mine[k] != stored[k]]
+        assert not bad, f"{key}: {', '.join(bad)} differ from the reference's"
+    else:
+        assert mine == stored, f"{key}: differs from the reference's answer"
+
+
+def result_fields(res, paired, skip=()):
+    """The fields assert_results_equal compares, as one dict of arrays: records, overlap records, corrected rows (bytes past a
+    read's length zeroed) and the counter block."""
+    out = {}
+    for o in ("out1", "out2") if paired else ("out1",):
+        for f in RESULT_FIELDS:
+            if f not in skip:
+                out[f"{o}.{f}"] = np.ascontiguousarray(res[o][f])
+    if paired and "ov" not in skip:
+        for f in ("overlapped", "has_gap", "offset", "overlap_len", "diff"):
+            out[f"ov.{f}"] = np.ascontiguousarray(res["ov"][f])
+    for k, a in res["arrs"].items():
+        if not k.startswith("len"):
+            ln = res["arrs"]["len" + k[-1]].astype(np.int64)
+            out[k] = np.where(np.arange(a.shape[1])[None, :] < ln[:, None], a, 0).astype(a.dtype)
+    out["counters"] = res["counters"].data
+    return out
+
+
+def check_result_reference(key, got, params, arrs, cycles, skip=(), nthreads=0):
+    """check_reference for a run_cpu / run_gpu result: the reference harness over the same batch is the answer."""
+    paired = bool(params.paired)
+    check_reference(key, result_fields(got, paired, skip),
+                    lambda: result_fields(run_cpu("ref", params, arrs, cycles, nthreads), paired, skip))
 
 
 def copy_arrays(arrs):

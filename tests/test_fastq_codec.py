@@ -7,29 +7,30 @@ import pytest
 import fp_testlib as T
 from fastp_b200 import capi
 
-needs_ref = pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 CASES = T.fastq_edge_cases()
 
 
-@needs_ref
+def ref_fastq_read_text(tmp_path, text, phred64=0):
+    path = tmp_path / "in.fq"
+    path.write_bytes(text)
+    return T.ref_fastq_read(path, phred64)
+
+
 @pytest.mark.reference
 @pytest.mark.parametrize("name", list(CASES))
 def test_oracle_decode_matches_fastqreader(tmp_path, name):
     text = CASES[name]
-    path = tmp_path / "in.fq"
-    path.write_bytes(text)
-    want = T.ref_fastq_read(path)
     d = T.oracle_fastq_decode(text, final=1, stride=512)
-    assert T.decoded_fields(text, d) == want, name
+    got = T.decoded_fields(text, d)
+    T.check_reference(f"fastq_decode/{name}", got, lambda: ref_fastq_read_text(tmp_path, text))
     if name in ("bad_strand", "empty_strand"):
-        assert d["info"]["error"] == 1 and d["info"]["error_record"] == len(want)
+        assert d["info"]["error"] == 1 and d["info"]["error_record"] == len(got)
     elif name == "length_mismatch":
         assert d["info"]["error"] == 2 and d["info"]["error_record"] == 1
     else:
         assert d["info"]["error"] == 0 and d["info"]["error_record"] == -1
 
 
-@needs_ref
 @pytest.mark.reference
 def test_oracle_decode_phred64_matches_fastqreader(tmp_path):
     rng = np.random.default_rng(3)
@@ -39,9 +40,8 @@ def test_oracle_decode_phred64_matches_fastqreader(tmp_path):
         s = "".join(rng.choice(list("ACGTN"), n)); q = bytes(rng.integers(59, 127, n).astype(np.uint8)).decode("latin1")
         recs.append(f"@p{i}\n{s}\n+\n{q}\n")
     text = "".join(recs).encode("latin1")
-    path = tmp_path / "p64.fq"; path.write_bytes(text)
     d = T.oracle_fastq_decode(text, final=1, phred64=1, stride=64)
-    assert T.decoded_fields(text, d) == T.ref_fastq_read(path, phred64=1)
+    T.check_reference("fastq_decode_phred64", T.decoded_fields(text, d), lambda: ref_fastq_read_text(tmp_path, text, phred64=1))
 
 
 @pytest.mark.parametrize("name", ["plain", "crlf", "blank_lines_between", "junk_before_name", "quality_starts_with_at", "long_names", "truncated_record"])
@@ -88,32 +88,24 @@ def test_capacity_limit_reports_more():
     assert d["info"]["n_records"] + d2["info"]["n_records"] == 40
 
 
-@needs_ref
 @pytest.mark.reference
 def test_oracle_decode_fuzz_matches_fastqreader(tmp_path):
     """300 random texts (mixed line ends, junk, broken records): same records as the reference's FastqReader."""
     rng = np.random.default_rng(2026)
     for k in range(300):
         text = T.fastq_fuzz_text(rng)
-        path = tmp_path / "f.fq"; path.write_bytes(text)
-        want = T.ref_fastq_read(path)
         got = T.decoded_fields(text, T.oracle_fastq_decode(text, final=1, stride=64))
-        assert got == want, (k, text)
+        T.check_reference(f"fastq_fuzz/{k}", got, lambda: ref_fastq_read_text(tmp_path, text))
 
 
-@needs_ref
 @pytest.mark.reference
 @pytest.mark.parametrize("paired", [1, 0])
 @pytest.mark.parametrize("case", ["default", "full"])
 def test_oracle_text_pipeline_equals_reference_cli(tmp_path, case, paired):
     """decode -> operator chain -> encode, all in the C port, against the UNMODIFIED reference CLI's output files: pins the whole
     text-path oracle (the -m gpu twin holds fp_fastq_process_host to the same files)."""
-    import os
     import test_gpu_fastq as G
-    if not os.path.exists(T.REF_CLI):
-        pytest.skip("oracle/_ref/fastp_ref not built")
     flags, p, t1, t2 = G.cli_inputs(case, paired, n=2000)
-    want = G.run_cli(tmp_path, flags, t1, t2)
     d1 = T.oracle_fastq_decode(t1, stride=160)
     arrs = {"seq1": d1["seq"].copy(), "qual1": d1["qual"].copy(), "len1": d1["len"].copy()}
     if paired:
@@ -123,4 +115,4 @@ def test_oracle_text_pipeline_equals_reference_cli(tmp_path, case, paired):
     got = [T.oracle_fastq_encode(t1, d1["recs"], res["out1"], res["arrs"]["seq1"], res["arrs"]["qual1"], 160)]
     if paired:
         got.append(T.oracle_fastq_encode(t2, d2["recs"], res["out2"], res["arrs"]["seq2"], res["arrs"]["qual2"], 160))
-    assert got == want
+    T.check_reference(f"cli_text/{case}/{paired}", got, lambda: G.run_cli(tmp_path, flags, t1, t2))

@@ -31,8 +31,26 @@ def synth_parallel(n, S, paired, profile, L, threads):
     return arrs
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("name,paired", [("cfg2_cut_right_polyg", 0), ("cfg3_overlap_correction", 1), ("cfg4_full", 1)])
+def reference_fields(p, arrs, paired, threads):
+    """records + counters + corrected rows of the reference's worker body over a copy of the rows, on `threads` host threads."""
+    n, S = arrs["seq1"].shape
+    a = {k: v.copy() for k, v in arrs.items()}
+    rb = capi.batch_from_arrays(a)
+    Lr = capi.make_layout(T.oracle(), paired, S, p.insert_size_max)
+    want_cnt = np.zeros(Lr.total, np.int64)
+    w1 = np.zeros(n, capi.READ_RESULT_DTYPE); w2 = np.zeros(n, capi.READ_RESULT_DTYPE); wov = np.zeros(n, capi.OV_RESULT_DTYPE)
+    rc = T.ref().fp_ref_process_mt(C.byref(p), C.byref(Lr), C.byref(rb), w1.ctypes.data, w2.ctypes.data if paired else None,
+                                   wov.ctypes.data if paired else None, want_cnt.ctypes.data, threads)
+    assert rc == 0
+    want = {"out1": w1, "out2": w2, "ov": wov, "counters": capi.CounterView(Lr, want_cnt), "arrs": a}
+    # adapter_pos is a device-side extra (where trimBySequence hit); the reference harness has no such field
+    return T.result_fields(want, paired, skip=("adapter_pos",))
+
+
+CASES = [("cfg2_cut_right_polyg", 0), ("cfg3_overlap_correction", 1), ("cfg4_full", 1)]
+
+
+@pytest.mark.parametrize("name,paired", CASES)
 def test_ten_million_units_equal_reference(name, paired):
     import torch
     if not torch.cuda.is_available():
@@ -42,15 +60,6 @@ def test_ten_million_units_equal_reference(name, paired):
     threads = len(os.sched_getaffinity(0))
     arrs = synth_parallel(n, S, paired, 1, L, min(threads, 32))
     p = T.config_params(name, paired, lib=T.oracle())
-    # reference: records + counters (rows are corrected in place -> work on a copy)
-    a = {k: v.copy() for k, v in arrs.items()}
-    rb = capi.batch_from_arrays(a)
-    Lr = capi.make_layout(T.oracle(), paired, S, p.insert_size_max)
-    want_cnt = np.zeros(Lr.total, np.int64)
-    w1 = np.zeros(n, capi.READ_RESULT_DTYPE); w2 = np.zeros(n, capi.READ_RESULT_DTYPE); wov = np.zeros(n, capi.OV_RESULT_DTYPE)
-    rc = T.ref().fp_ref_process_mt(C.byref(p), C.byref(Lr), C.byref(rb), w1.ctypes.data, w2.ctypes.data if paired else None,
-                                   wov.ctypes.data if paired else None, want_cnt.ctypes.data, threads)
-    assert rc == 0
     # CUDA: HBM-resident, one launch
     ctx = fp_gpu.GpuCtx(p, 1 << 18, S, S)
     t = {k: torch.from_numpy(v).cuda() for k, v in arrs.items()}
@@ -66,8 +75,7 @@ def test_ten_million_units_equal_reference(name, paired):
     torch.cuda.synchronize()
     got = {"out1": o1.cpu().numpy().view(capi.READ_RESULT_DTYPE), "out2": o2.cpu().numpy().view(capi.READ_RESULT_DTYPE)[:n if paired else 0],
            "ov": ov.cpu().numpy().view(capi.OV_RESULT_DTYPE)[:n if paired else 0], "counters": ctx.counters(),
-           "arrs": {k: v.cpu().numpy().reshape(arrs[k].shape) for k, v in t.items()}, "layout": ctx.L}
-    want = {"out1": w1, "out2": w2, "ov": wov, "counters": capi.CounterView(Lr, want_cnt), "arrs": a, "layout": Lr}
-    # adapter_pos is a device-side extra (where trimBySequence hit); the reference harness has no such field
-    T.assert_results_equal(got, want, paired, skip=("adapter_pos",), what=f"{name} {n} units")
+           "arrs": {k: v.cpu().numpy().reshape(arrs[k].shape) for k, v in t.items()}}
     ctx.close()
+    del t
+    T.check_reference(f"scale/{name}/{n}", T.result_fields(got, paired, skip=("adapter_pos",)), lambda: reference_fields(p, arrs, paired, threads))

@@ -21,22 +21,26 @@ def host_candidates(seq, lens, stride, seqlen):
     return c
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("L,S,profile,n", [(250, 256, 3, 7000), (150, 160, 1, 4000), (100, 112, 3, 3000)])
-def test_candidates_equal_reference_evaluator(tmp_path, L, S, profile, n):
-    _, arrs = T.synth_host(n, S, 1, 0, 42, profile, L)
+def reference_candidates(tmp_path, arrs, side, L):
+    """Evaluator::computeOverRepSeq of the reference over the same reads written as FASTQ."""
     ref = T.ref()
     ref.fp_ref_compute_overrep.restype = C.c_int
     ref.fp_ref_compute_overrep.argtypes = [C.c_char_p, C.c_int, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]
+    fn = os.path.join(tmp_path, f"r{side}.fq")
+    open(fn, "wb").write(T.fastq_text(arrs["seq" + side], arrs["qual" + side], arrs["len" + side], side))
+    out = C.create_string_buffer(1 << 22); used = C.c_int64()
+    k = ref.fp_ref_compute_overrep(fn.encode(), L, out, len(out), C.byref(used))
+    want = out.raw[:used.value].split(b"\0")[:-1]
+    assert k == len(want)
+    return want
+
+
+@pytest.mark.parametrize("L,S,profile,n", [(250, 256, 3, 7000), (150, 160, 1, 4000), (100, 112, 3, 3000)])
+def test_candidates_equal_reference_evaluator(tmp_path, L, S, profile, n):
+    _, arrs = T.synth_host(n, S, 1, 0, 42, profile, L)
     for side in "12":
         got = host_candidates(arrs["seq" + side], arrs["len" + side], S, L)
-        fn = os.path.join(tmp_path, f"r{side}.fq")
-        open(fn, "wb").write(T.fastq_text(arrs["seq" + side], arrs["qual" + side], arrs["len" + side], side))
-        out = C.create_string_buffer(1 << 22); used = C.c_int64()
-        k = ref.fp_ref_compute_overrep(fn.encode(), L, out, len(out), C.byref(used))
-        want = out.raw[:used.value].split(b"\0")[:-1]
-        assert k == len(want)
-        assert got == want, (len(got), len(want))
+        T.check_reference(f"overrep_prescan/{L}/{side}", got, lambda: reference_candidates(tmp_path, arrs, side, L))
     if profile == 3:
         assert len(got) > 0          # the planted sequences are found
 
